@@ -2,7 +2,7 @@
 """bench.py -- tokens/sec of the LSTM-LM train step (main.py:109-117) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config large|medium|small]
-                    [--impl ours|reference] [--engine tc|simt]
+                    [--impl ours|reference] [--engine tc|simt] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one synthetic
 [T,B] window per GPU: forward, softmax-NLL, backward, (gradient all-reduce when N>1),
@@ -190,14 +190,37 @@ def cpu_port_leg(c, budget_s, steps=None, warmup=1):
             "host_cpus": os.cpu_count()}, dt
 
 
+DUMP_SAMPLE = 1 << 20       # elements kept of a larger parameter tensor: the Large config dumps ~25 MB
+
+
+def dump_outputs(out_dir, tr):
+    """Write what the last train step handed its caller as float32 .npy files: loss, clip norm, the carried (h, c)
+    states and the updated parameters.  A parameter tensor of more than DUMP_SAMPLE elements is cut to a sample at
+    fixed, seeded positions, the same in every run of the same config, so two builds compare element for element.
+    Compare over few steps: fp32 atomics add in another order from run to run and the carried states amplify that
+    (two runs of one build, Large, B200 at 1000 W: 2e-4 of a tensor's scale at --steps 1, 1e-3 at 10, 0.2 at 50)."""
+    import numpy as np
+    arrays = {"loss": tr.loss, "norm": tr.norm}
+    for l, (h, c) in enumerate(tr.states):
+        arrays[f"state_h{l}"], arrays[f"state_c{l}"] = h, c
+    for k, p in tr.model.named_parameters():
+        arrays["param_" + k] = p
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, total
+
+
 def run_reference(args, c, name):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # bounded sample: at most ~100 s of CPU work whatever --steps says (0.73 s/step for Large on 64 threads)
-    probe, dt1 = cpu_port_leg(c, 0, steps=1, warmup=1)
-    run_steps = max(3, min(args.steps, int(100.0 / max(dt1, 1e-3))))
-    base, dt = cpu_port_leg(c, 0, steps=run_steps, warmup=min(max(1, args.warmup), 3))
+    base, dt = cpu_port_leg(c, 0, steps=args.steps, warmup=args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": "tokens/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -269,6 +292,8 @@ def run_ours(args, c, name):
     dev_ms, _, launches = timed_region(lambda x, y: tr.train_step(x, y, c["lr"], c["clip"]), dev_batches)
     clocks = sampler.stop() if sampler else None
     loss_after = tr.loss.item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr)
     # replica check: after the timed steps every rank must hold bit-identical parameters (same all-reduced
     # gradients, same clip, same update) -- MAX - MIN over ranks of two checksums, must be 0
     dp_check = None
@@ -398,7 +423,14 @@ def main():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--strict-update", action="store_true",
                     help="apply every weight update at the end of its own step (no lazy update beside the next forward)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last step's loss, norm, states and (sampled) parameters "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     c = CONFIGS[args.config]
     if args.impl == "reference":
